@@ -17,6 +17,11 @@ and every step touches fresh random rows, so no explicit L2 flush is needed
 ("inputs larger than L2").  `e2e` times the same K steps through the public
 API (`sess.run`) with per-step H2D of the batch from pinned memory and a D2H
 read of the loss.
+
+`--dump-outputs DIR` writes what the last timed step returned (loss and final LSTM
+state for LM1B) as .npy files: the inputs and weights are seeded, so two builds run with
+the same arguments can be compared output for output.  The benchmark writes nothing into
+the source tree, which may be read-only.
 """
 import argparse
 import json
@@ -26,6 +31,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True        # no __pycache__ in a possibly read-only tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -61,7 +67,51 @@ def parse():
                     help="with --no-extras: still report the graph-replayed comm probes")
     ap.add_argument("--sustained-s", type=float, default=3.0,
                     help="length of the additional sustained-clock run (seconds)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned "
+                         "(rank 0) as DIR/<name>.npy, at most 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out, path, limit=DUMP_LIMIT_BYTES):
+    """Write the arrays of one step's result as `path/<name>.npy`.  Floating arrays are
+    stored as float32 (float64 stays float64), integer and boolean ones as float64.  The
+    files stay under `limit` bytes in all: the budget is shared out smallest array first,
+    and an array larger than its share is replaced by the elements of its flattened form at
+    sorted indices drawn with a fixed seed, so every run samples the same positions.
+    Returns {name: {"shape": original shape, "stored": elements written}}."""
+    import re
+    import numpy as np
+    import torch
+    arrays = {}
+    for name, v in out.items():
+        if torch.is_tensor(v):
+            v = v.detach()
+            v = v.float() if v.is_floating_point() and v.dtype != torch.float64 else v.double()
+            arrays[name] = v.cpu().numpy()
+        elif isinstance(v, (bool, int, float)):
+            arrays[name] = np.asarray(v, dtype=np.float64)
+    os.makedirs(path, exist_ok=True)
+    left, written = limit, {}
+    for i, name in enumerate(sorted(arrays, key=lambda k: (arrays[k].nbytes, k))):
+        a = arrays[name]
+        shape = list(a.shape)
+        share = left // (len(arrays) - i) - 1024          # room for the .npy header
+        if a.nbytes > share:
+            n = max(share // a.itemsize, 0)
+            idx = np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))
+            a = a.reshape(-1)[idx]
+        fn = os.path.join(path, re.sub(r"[^A-Za-z0-9_.-]", "_", name) + ".npy")
+        np.save(fn, a)
+        left -= os.path.getsize(fn)
+        written[name] = {"shape": shape, "stored": int(a.size)}
+    return written
 
 
 class ClockSampler(object):
@@ -248,9 +298,11 @@ def _max_over_ranks(torch, dist, world, dev, vals):
 
 
 def measure(args, model, dtype, K, Wm, world, rank, protocol="nvlink", e2e=True,
-            comm_stamps=False, sustained_s=0.0, sampler=None):
+            comm_stamps=False, sustained_s=0.0, sampler=None, dump_dir=None):
     """Build a session for `model`, run Wm warm-up + exactly K timed steps (device events,
-    max over ranks) and the optional extra regions; returns the result block."""
+    max over ranks) and the optional extra regions; returns the result block.  With
+    `dump_dir`, rank 0 writes the last timed step's result there before any later step
+    runs (a replayed CUDA graph returns the same tensors every step)."""
     import torch
     import torch.distributed as dist
     import parallax_b200 as parallax
@@ -304,6 +356,8 @@ def measure(args, model, dtype, K, Wm, world, rank, protocol="nvlink", e2e=True,
            "cuda_graph": bool(getattr(eng, "graph_captured", False)),
            "run_option": eng.run_option.lower(), "protocol": protocol,
            "_desc": desc, "_baseline": baseline, "_window": (t_w0, t_w1)}
+    if dump_dir is not None and rank == 0:
+        res["dump_outputs"] = {"dir": dump_dir, "arrays": dump_outputs(out, dump_dir)}
 
     # ---- sustained run: the same step for >= sustained_s seconds -------------
     if sustained_s > 0:
@@ -417,7 +471,8 @@ def main():
     main_blk = measure(args, args.model, args.dtype, K, Wm, world, rank,
                        protocol=args.protocol, e2e=not args.no_e2e,
                        comm_stamps=extras or args.comm,
-                       sustained_s=args.sustained_s if extras else 0.0, sampler=sampler)
+                       sustained_s=args.sustained_s if extras else 0.0, sampler=sampler,
+                       dump_dir=args.dump_outputs)
     clocks = sampler.window(*main_blk["_window"]) if rank == 0 else None
     blocks = {}
     if extras and args.model == "lm1b":
@@ -472,6 +527,8 @@ def main():
             "sustained": main_blk.get("sustained"), "loss": main_blk["loss"],
             "selfcheck": selfcheck,
         }
+        if "dump_outputs" in main_blk:
+            rec["dump_outputs"] = main_blk["dump_outputs"]
         rec.update(blocks)
         print(json.dumps(rec))
     comm.shutdown()

@@ -18,9 +18,12 @@ def _free_port():
 
 
 def _entry(rank, world, port, fn, args, outdir, env):
+    # the ranks are CPU processes: with a GPU visible every rank would pick NCCL on the
+    # same device, which NCCL refuses (CUDA is first initialised after this line)
     os.environ.update({"RANK": str(rank), "WORLD_SIZE": str(world),
                        "LOCAL_RANK": str(rank), "MASTER_ADDR": "127.0.0.1",
-                       "MASTER_PORT": str(port), "OMP_NUM_THREADS": "1"})
+                       "MASTER_PORT": str(port), "OMP_NUM_THREADS": "1",
+                       "CUDA_VISIBLE_DEVICES": ""})
     os.environ.update(env or {})
     import torch
     torch.set_num_threads(1)

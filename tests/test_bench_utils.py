@@ -1,5 +1,6 @@
 """bench.py host-side pieces that can be checked without a GPU: the clock sampler
-(against a fake `nvidia-smi`), the reference arm's one-line contract."""
+(against a fake `nvidia-smi`), the reference arm's one-line contract, the output dump and
+the argument checks."""
 import json
 import os
 import stat
@@ -66,3 +67,38 @@ def test_reference_arm_prints_one_json_line_per_job():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference",
                         "--gpus", "2"], env=env, capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_types_names_and_size_limit(tmp_path):
+    import numpy as np
+    import torch
+    import bench
+    out = {"loss": torch.tensor(2.5), "state/h": torch.ones(3, 4, dtype=torch.bfloat16),
+           "ids": torch.arange(5), "big": torch.arange(40000, dtype=torch.float64),
+           "step": 7, "note": "not an array"}
+    got = bench.dump_outputs(out, str(tmp_path / "a"), limit=64 << 10)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["big.npy", "ids.npy", "loss.npy", "state_h.npy", "step.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 10
+    loss = np.load(tmp_path / "a" / "loss.npy")
+    assert loss.dtype == np.float32 and loss.shape == () and float(loss) == 2.5
+    h = np.load(tmp_path / "a" / "state_h.npy")
+    assert h.dtype == np.float32 and h.shape == (3, 4) and (h == 1).all()
+    assert np.load(tmp_path / "a" / "ids.npy").dtype == np.float64
+    assert float(np.load(tmp_path / "a" / "step.npy")) == 7.0
+    # the large array is a sample of its elements: same positions on every call
+    big = np.load(tmp_path / "a" / "big.npy")
+    assert got["big"]["shape"] == [40000] and got["big"]["stored"] == big.size < 40000
+    assert (np.diff(big) > 0).all() and (big == big.astype(np.int64)).all()
+    bench.dump_outputs(out, str(tmp_path / "b"), limit=64 << 10)
+    assert (np.load(tmp_path / "b" / "big.npy") == big).all()
+    # under the limit nothing is sampled
+    got = bench.dump_outputs({"big": out["big"]}, str(tmp_path / "c"))
+    assert got["big"]["stored"] == 40000
+    assert (np.load(tmp_path / "c" / "big.npy") == np.arange(40000)).all()
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
